@@ -20,6 +20,7 @@ download).  Extra objects on the same JSON line:
     python bench.py --gpus N --steps K --warmup W            # torchrun for N > 1
     python bench.py --impl reference ...                       # CPU oracle arm (rank 0 only)
     python bench.py --quick                                    # headline legs only (A/B runs)
+    python bench.py --dump-outputs DIR                         # also write the headline window's solved parameters as .npy
 """
 import argparse
 import ctypes
@@ -189,6 +190,13 @@ def kernel_split(lvb, run, iters):
     return {k: v / iters for k, v in acc.items()}
 
 
+def dump_outputs(out_dir, problem):
+    """What Problem.solve hands back to its caller: the solved parameter blocks (about 33 kB at configs[1])."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("poses", problem.poses()), ("vec3", problem.vec3()), ("inv_depths", problem.inv_depths())):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -201,6 +209,8 @@ def main():
     ap.add_argument("--skip-global", action="store_true")
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--blocks", type=int, default=0, help="repetitions of the timed region (0: enough for >= 50 solves); profiler runs use 1")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of the headline window returns to a caller "
+                    "(poses, vec3, inverse depths of rank 0's shard) as DIR/<name>.npy in float64, to compare builds output for output")
     args = ap.parse_args()
     if args.quick:
         args.skip_icp = args.skip_roofline = args.skip_global = args.skip_cpu = True
@@ -307,6 +317,9 @@ def main():
         sampler.start()
         w10 = window_leg(ctx, N_KF, N_LM, args.steps, args.warmup)
         sampler.stop_flag = True
+        if args.dump_outputs and rank == 0:
+            # the problem still holds the state its last timed solve left (the e2e part of the leg solves fresh problems)
+            dump_outputs(args.dump_outputs, w10["problem"])
         value = w10["rows"] * w10["iters"] / (w10["ms"] * 1e-3)
         line = {
             "metric": "ba_residual_jacobian_rows_per_s", "value": value, "unit": "rows/s", "n_gpus": world, "steps": w10["iters"], "warmup": args.warmup,

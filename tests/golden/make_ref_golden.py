@@ -206,6 +206,86 @@ def assoc_case(kind):
     return sc
 
 
+BACKEND_MODES = (0, 1, 2, 3, 4)       # tests/cpp/ref_backend_dropin.cpp: window + IMU, visual only, FullBA, Initializer, Environment
+
+
+def _parse_ba_record(raw):
+    """The log of oracle/ref_record.cpp -> one dict per solve: the problem as the C ABI received it, the options (the fields
+    of lvb_solve_options in order), and the oracle's summary (rc, initial cost, final cost, iterations, successful steps,
+    termination) and solved blocks."""
+    from lvio_fusion_b200.backend import CONST_STRIDE, IDX_STRIDE
+    off, solves, cur = 0, [], None
+
+    def take(dtype, n):
+        nonlocal off
+        a = np.frombuffer(raw, dtype=dtype, count=n, offset=off).copy()
+        off += a.nbytes
+        return a
+    while off < len(raw):
+        tag = int(take(np.int32, 1)[0])
+        if tag == 1:
+            cur = {"loss": np.zeros(6)}
+        elif tag == 2:
+            cur["cameras"] = take(np.float64, 22)
+        elif tag in (3, 4, 5):
+            name, w = {3: ("poses", 7), 4: ("vec3", 3), 5: ("rho", 1)}[tag]
+            n = int(take(np.int32, 1)[0])
+            cur[name] = take(np.float64, n * w).reshape(n, w) if w > 1 else take(np.float64, n)
+            cur[name + "_const"] = take(np.uint8, n) if take(np.int32, 1)[0] else np.zeros(n, np.uint8)
+        elif tag == 6:
+            kind, n = (int(v) for v in take(np.int32, 2))
+            cur["f%d_consts" % kind] = take(np.float64, n * CONST_STRIDE[kind]).reshape(n, CONST_STRIDE[kind])
+            cur["f%d_idx" % kind] = take(np.int32, n * IDX_STRIDE[kind]).reshape(n, IDX_STRIDE[kind])
+        elif tag == 7:
+            kind = int(take(np.int32, 1)[0])
+            cur["loss"][kind] = take(np.float64, 1)[0]
+        elif tag == 8:
+            cur["options"], cur["summary"] = take(np.float64, 10), take(np.float64, 6)
+            for name, w in (("poses", 7), ("vec3", 3), ("rho", 1)):
+                cur["out_" + name] = take(np.float64, len(cur[name]) * w).reshape(cur[name].shape)
+            solves.append(cur)
+        else:
+            raise ValueError("bad record tag %d" % tag)
+    return solves
+
+
+def _harness_values(stdout):
+    """`tag key value key value ...` lines of the drop-in harness -> {"tag.key": value} for the numeric ones."""
+    rec = {}
+    for line in stdout.splitlines():
+        t = line.split()
+        for k, v in zip(t[1::2], t[2::2]):
+            try:
+                rec[t[0] + "." + k] = float(v)
+            except ValueError:
+                pass
+    return rec
+
+
+def run_reference_backend():
+    """Every bundle-adjustment problem the reference's Backend::BuildProblem / adapt::Solve, imu::FullBA, Initializer and
+    Environment::Optimize (tests/cpp/ref_backend_dropin.cpp, compiled in place) hand to the solver through the product shim, as
+    the oracle received and solved it; with the cost the reference's own functors assign to the problems of modes 0 and 1
+    (ref_backend_truth) and the harness' error summary before and after (ref_backend_orc)."""
+    ref = os.path.join(ROOT, "oracle", "_ref")
+    out = {}
+    for mode in BACKEND_MODES:
+        with tempfile.TemporaryDirectory() as td:
+            log = os.path.join(td, "ba.log")
+            env = dict(os.environ, LVB_RECORD=log, LD_PRELOAD=os.path.join(ref, "ref_record.so"))
+            orc = _harness_values(subprocess.run([os.path.join(ref, "ref_backend_orc"), str(mode)], env=env, check=True, capture_output=True, text=True).stdout)
+            with open(log, "rb") as f:
+                solves = _parse_ba_record(f.read())
+        out["m%d_n_solves" % mode] = np.array(len(solves))
+        for j, s in enumerate(solves):
+            out.update({"m%d_s%d_%s" % (mode, j, k): v for k, v in s.items()})
+        out["m%d_rel" % mode] = np.array([orc.get(k, np.nan) for k in ("before.rel_t", "before.rel_r", "after.rel_t", "after.rel_r")])
+        if mode < 2:
+            truth = _harness_values(subprocess.run([os.path.join(ref, "ref_backend_truth"), str(mode)], check=True, capture_output=True, text=True).stdout)
+            out["m%d_reference_initial_cost" % mode] = np.array(truth["reference.initial_cost"])
+    return out
+
+
 def main():
     if not os.path.isdir("/root/reference"):
         raise SystemExit("the reference tree is not mounted here; the committed fixture stays as it is")
@@ -226,6 +306,9 @@ def main():
         out.update({kind + "_head": head, kind + "_table": tab, kind + "_e0": np.asarray(e0)})
         print("reference scan-to-map (%s): %d blocks of %d scan points, prior weight %.3f, huber %.2f" % (kind, int(head[0]), len(tab), head[2], head[3]))
     np.savez_compressed(os.path.join(HERE, "ref_assoc.npz"), **out)
+    ba = run_reference_backend()
+    np.savez_compressed(os.path.join(HERE, "ref_backend.npz"), **ba)
+    print("reference backend problems written:", {m: int(ba["m%d_n_solves" % m]) for m in BACKEND_MODES})
 
 
 if __name__ == "__main__":
